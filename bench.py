@@ -6,6 +6,7 @@ minibatch-OT couplings/sec (N=8192, d=784) [+ ODE samples/sec], 1..8 B200 of one
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's coupled batch to DIR/*.npy
 
 One step = one full coupling `OTPlanSampler("sinkhorn", reg=0.05, normalize_cost=True).sample_plan`
 (cost matrix + 100 log-domain Sinkhorn iterations, stopThr=0 + N pair draws + gather) on a
@@ -208,7 +209,13 @@ def main():
     ap.add_argument("--no-ode", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the c1/c4/c5 sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0's sample_plan pair "
+                         "x0[i], x1[j], float32) as DIR/<name>.npy: the same arguments give the same inputs and draws, "
+                         "so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "cfm_b200":
+        ap.error("--dump-outputs writes the outputs of the cfm_b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "cfm_b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -303,6 +310,10 @@ def main():
     elapsed_ms = max_over_ranks(elapsed_ms)
     value = world * args.steps / (elapsed_ms * 1e-3)
     assert out[0].shape == (N, D) and out[0].is_cuda
+    if args.dump_outputs and rank == 0:  # 2 x 8192 x 784 float32 = 51 MB
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in zip(("x0_coupled", "x1_coupled"), out):
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), t.float().cpu().numpy())
 
     # ---- parity gate reported with the number: marginals of the implied plan (float64, device)
     cp = sampler._couple(x0, x1, dev)

@@ -2,11 +2,10 @@
 
 Functional restatement (numpy / torch-CPU / scipy) of what
 ``torchcfm.optimal_transport.OTPlanSampler`` does around the POT solver, so that
-the parity tests and bench.py's CPU baseline can run on the GPU box where
-/root/reference is not mounted.  Every function cites the reference lines it
-follows.  tests/test_oracle.py checks this file against the unmodified reference
-package (imported from /root/reference on top of oracle/ot) whenever that tree is
-present, and against the committed fixtures in tests/golden/ otherwise.
+the parity tests and bench.py's CPU baseline can run where the reference
+package is not installed.  Every function cites the reference lines it
+follows.  tests/test_oracle.py checks this file against the committed fixtures in
+tests/golden/, which the unmodified reference package (on top of oracle/ot) wrote.
 
 PARITY STATUS: exact-OT pinned (scipy LSA, reference tests, golden fixtures
 generated from the reference glue).  Sinkhorn plan values: parity unpinned at the

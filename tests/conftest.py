@@ -8,7 +8,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE = "/root/reference"
 GOLDEN = os.path.join(ROOT, "tests", "golden", "reference_vectors.npz")
 
 

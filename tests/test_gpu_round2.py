@@ -235,7 +235,7 @@ def _x10k():
 
 
 @pytest.mark.parametrize("fused", [1, 0])
-def test_mlp_b10000_tensor_core_vs_reference_vectors(fused):
+def test_mlp_b10000_tensor_core_vs_reference_vectors(fused, tmp_path):
     """BASELINE config 3's forward at the full batch through the tcgen05 paths -- the fused persistent kernel
     and the per-layer launches -- against vectors generated by the unmodified reference MLP
     (tests/golden/make_golden_mlp10k.py): 96 whole rows, all row sums, all column sums.  Gate: 1e-5 of max|y|."""
@@ -259,7 +259,7 @@ def test_mlp_b10000_tensor_core_vs_reference_vectors(fused):
                 y = m.vector_field(0.37, x)
             np.save(sys.argv[1], y.cpu().numpy())
         """ % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-        out = "/tmp/mlp10k_perlayer.npy"
+        out = str(tmp_path / "mlp10k_perlayer.npy")
         env = dict(os.environ, CFM_MLP_FUSED="0")
         subprocess.run([sys.executable, "-c", code, out], check=True, env=env, timeout=300)
         y = np.load(out).astype(np.float64)
